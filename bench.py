@@ -25,6 +25,11 @@ into the node's POSIX shared-memory segment in the reference's byte layout.
 Launch: python bench.py [--gpus N --steps K --warmup W] ; for N>1 under
 torch.distributed.run, one rank per GPU, every rank saves its own 16 GB shard
 (weak scaling, no data-path collective).
+
+--dump-outputs DIR: rank 0 writes what its timed legs left in their segments after the
+last timed step — raw_segment.npy (leg 1) and checkpoint_segment.npy (leg 2; the
+reference arm writes its own segment under that name) — so that two builds can be
+compared output for output on the same seeded inputs.
 """
 
 from __future__ import annotations
@@ -53,7 +58,32 @@ def parse():
     ap.add_argument("--scale", type=float, default=float(os.getenv("BENCH_SCALE", "1.0")),
                     help="shrink dim 0 of every 2-D tensor (debug only; 1.0 = BASELINE config)")
     ap.add_argument("--no-stall", action="store_true", help="skip the stall measurement")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write a seeded sample of each segment the "
+                         "timed path filled in its last step as DIR/<name>.npy (float32)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+DUMP_WORDS = 4 << 20  # 16-bit words sampled per dumped segment: 16 MB of float32 each
+
+
+def dump_segment(out_dir: str, name: str, buf) -> None:
+    """Writes the 16-bit words of `buf` (bf16 payload) widened bit-exactly to float32 as
+    out_dir/name.npy: all of them for a small segment, else DUMP_WORDS at positions drawn
+    from a fixed seed, so that two builds of the same workload dump the same positions."""
+    import numpy as np
+
+    words = np.frombuffer(buf, dtype=np.uint16, count=len(buf) // 2)
+    if words.size > DUMP_WORDS:
+        pos = np.sort(np.random.default_rng(20240601).integers(0, words.size, DUMP_WORDS))
+        words = words[pos]
+    out = (words.astype(np.uint32) << 16).view(np.float32)
+    del words
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, name + ".npy"), out)
 
 
 class ClockSampler:
@@ -249,6 +279,9 @@ def run_reference(args):
         dt_mine = time.perf_counter() - t0
         barrier_sync(world)
         dt = max_over_ranks(dt_mine, world, dev)
+        if args.dump_outputs and rank == 0:
+            dump_segment(args.dump_outputs, "checkpoint_segment",
+                         saver.buf if kind == "reference" else saver.segment.buf)
         # restore the reference's way: CPU views on the (pageable) segment, one
         # H2D copy_ per tensor (ckpt_saver.py:144-161 + model.load_state_dict)
         views = reference_views(saver, kind)
@@ -456,6 +489,8 @@ def run_ours(args):
         want = t.view(-1).view(torch.uint8)[:n].cpu().numpy()
         assert np.array_equal(img[off:off + n], want), "segment image mismatch"
     del img
+    if args.dump_outputs and rank == 0:
+        dump_segment(args.dump_outputs, "raw_segment", seg)
     plan.destroy()
     ctx.host_unregister(addr)
     seg.close()
@@ -483,6 +518,9 @@ def run_ours(args):
     barrier_sync(world)
     e2e_ms = (time.perf_counter() - t0) * 1e3
     k3, _ = ctx.launch_count()
+    if args.dump_outputs and rank == 0:
+        dump_segment(args.dump_outputs, "checkpoint_segment",
+                     ckpt.engine._shm_handler.shared_memory.buf)
     e2e_ms = max_over_ranks(e2e_ms, world, dev)
     e2e = S * world * args.steps / e2e_ms / 1e6
     api_timings = ckpt.engine.last_save_timings()

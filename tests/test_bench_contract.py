@@ -74,3 +74,30 @@ def test_reference_arm_line():
     assert {"value", "unit", "h2d_bytes_per_step", "d2h_bytes_per_step"} <= set(d["e2e"])
     assert d["e2e"]["value"] == d["value"]
     assert {"kind", "cores", "sample", "value"} <= set(d["cpu_baseline"])
+
+
+def test_dump_segment_is_bit_exact_seeded_and_bounded(tmp_path, monkeypatch):
+    """--dump-outputs: bf16 words come back widened bit-exactly to float32; a segment larger
+    than the sample is sampled at the same positions every time."""
+    import sys
+
+    import numpy as np
+    import torch
+
+    sys.path.insert(0, ROOT)
+    import bench
+
+    t = torch.randn(1000, dtype=torch.float32).to(torch.bfloat16)
+    buf = bytearray(t.view(torch.uint16).numpy().tobytes())
+    bench.dump_segment(str(tmp_path / "a"), "seg", buf)
+    got = np.load(tmp_path / "a" / "seg.npy")
+    assert got.dtype == np.float32 and np.array_equal(got, t.float().numpy())
+
+    monkeypatch.setattr(bench, "DUMP_WORDS", 64)
+    big = bytearray(np.arange(5000, dtype=np.uint16).tobytes())
+    for d in ("b", "c"):
+        bench.dump_segment(str(tmp_path / d), "seg", big)
+    b, c = np.load(tmp_path / "b" / "seg.npy"), np.load(tmp_path / "c" / "seg.npy")
+    assert b.shape == (64,) and np.array_equal(b.view(np.uint32), c.view(np.uint32))
+    words = b.view(np.uint32) >> 16
+    assert np.all(np.diff(words.astype(np.int64)) >= 0) and words.max() < 5000

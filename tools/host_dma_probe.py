@@ -7,8 +7,8 @@ all ranks at once; prints per-rank and aggregate GB/s per kind.
   tmpfs_nonuma same, FC_NO_NUMA=1
   hostalloc    cudaHostAlloc (torch pin_memory)
   anon_thp     anonymous mmap + MADV_HUGEPAGE, registered the same way
-  tmpfs_thp    tmpfs with transparent_hugepage/shmem_enabled=advise, if this process may
-               write that knob (restored afterwards)
+
+The host's transparent-hugepage settings are reported as found; the probe never changes them.
 """
 import json
 import mmap
@@ -34,7 +34,6 @@ REPS = 3
 ctx = native.get_context(local)
 src = torch.empty(SIZE, dtype=torch.uint8, device=dev)
 src.random_(0, 255)
-THP_KNOB = "/sys/kernel/mm/transparent_hugepage/shmem_enabled"
 
 
 def meminfo(*keys):
@@ -135,26 +134,6 @@ run_tmpfs("tmpfs_nonuma", {"FC_NO_NUMA": "1"})
 run_hostalloc()
 run_anon_thp()
 
-# shmem THP, if we may flip the knob
-old = None
-flag = torch.zeros(1, device=dev)
-if rank == 0:
-    try:
-        cur = open(THP_KNOB).read()
-        old = cur[cur.index("[") + 1:cur.index("]")]
-        open(THP_KNOB, "w").write("advise")
-        flag += 1
-    except Exception as e:  # read-only /sys in a container
-        print(json.dumps({"kind": "tmpfs_thp", "skipped": f"{type(e).__name__}: {e}"}), flush=True)
-if world > 1:
-    dist.broadcast(flag, 0)
-if flag.item() > 0:
-    try:
-        run_tmpfs("tmpfs_thp")
-    finally:
-        barrier()
-        if rank == 0 and old is not None:
-            open(THP_KNOB, "w").write(old)
 if rank == 0:
     print(json.dumps({"thp": {k: open(f"/sys/kernel/mm/transparent_hugepage/{k}").read().strip()
                               for k in ("enabled", "shmem_enabled", "defrag")},
